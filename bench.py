@@ -223,13 +223,10 @@ def cpu_rate(cfg, sample_clips=1, steps=1, warmup=0):
     return sample_clips * steps / dt, dt / steps
 
 
-REFERENCE_BUDGET_S = float(os.environ.get("PASST_REF_BUDGET_S", "150"))
-
-
 def run_reference(args, rank, world):
-    """Reference arm: the reference algorithm (oracle port, bit-exact with /root/reference on CPU) on the host cores.
-    One step = one full step of the configuration on a bounded 1-clip sample; at most --steps steps are timed, fewer
-    if the time budget (a few minutes) would be exceeded — the number actually timed is reported as `steps`."""
+    """Reference arm: the reference algorithm (oracle port, bit-exact with the reference on CPU) on the host cores.
+    One step = one full step of the configuration on a bounded 1-clip sample; exactly --steps steps are timed after
+    min(--warmup, 5) warm-up steps, so a run's last step (and --dump-outputs) does not depend on the host's speed."""
     if rank != 0:
         return
     cfg = CONFIGS[args.config]
@@ -240,16 +237,11 @@ def run_reference(args, rank, world):
     warm = min(max(0, args.warmup), 5)
     for _ in range(warm):
         step()
-        if time.perf_counter() - t_start > 0.3 * REFERENCE_BUDGET_S:
-            break
     warm_s = time.perf_counter() - t_start
     done, t0 = 0, time.perf_counter()
-    while done < max(1, args.steps):
-        step()
+    while done < args.steps:
+        result = step()
         done += 1
-        elapsed = time.perf_counter() - t0
-        if (time.perf_counter() - t_start) + elapsed / done > REFERENCE_BUDGET_S:
-            break
     dt = time.perf_counter() - t0
     rate = sample * done / dt
     what = "train step (mel train + fwd + bwd + AdamW)" if cfg["kind"] == "train" else "forward (mel eval + net eval)"
@@ -260,12 +252,14 @@ def run_reference(args, rank, world):
         "data": "synthetic",
         "config": {"workload": cfg["workload"], "name": args.config,
                    "sample": f"{sample} clip per step on the host CPU ({CPU_THREADS} threads)",
-                   "requested_steps": args.steps, "time_budget_s": REFERENCE_BUDGET_S, "warmup_s": warm_s},
+                   "requested_steps": args.steps, "warmup_s": warm_s},
         "cpu_baseline": {"value": rate, "unit": "clips/s", "cores": CPU_THREADS, "kind": "port",
                          "sample": f"{done} x {sample}-clip {what}, oracle port, fp32"},
         "e2e": {"value": rate, "unit": "clips/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        _write_outputs(args.dump_outputs, {"loss" if cfg["kind"] == "train" else "logits": result})
     _emit(line)
 
 
@@ -449,8 +443,15 @@ def run_candidate(args, rank, local_rank, world):
     if rank == 0:
         sampler.start()
     L.reset_launch_count()
-    ms_dev = timed(lambda i: run_step(dev_waves[i % n_batches]), args.steps)
+    last = [None]
+
+    def timed_step(i):
+        last[0] = run_step(dev_waves[i % n_batches])
+
+    ms_dev = timed(timed_step, args.steps)
     launches = L.launch_count()
+    # taken before anything below runs another step on the same weights
+    dumped = _timed_outputs(net, last[0], train) if (args.dump_outputs and rank == 0) else None
     if graphed is not None:
         # kernels are replayed by the graph; count the launches of one eager step and scale
         L.reset_launch_count()
@@ -589,8 +590,46 @@ def run_candidate(args, rank, local_rank, world):
                 sb = stock_gpu_block(cfg, B, steps=min(args.steps, 20))
                 line["stock_gpu"] = sb
                 line["vs_stock"] = value / sb["best_clips_per_s"] if sb["best_clips_per_s"] else None
+        if dumped is not None:
+            _write_outputs(args.dump_outputs, dumped)
         _emit(line)
     return line
+
+
+DUMP_SAMPLE = 1 << 20      # elements in a sampled output (4 MB as float32)
+
+
+def _seeded_sample(tensors, n=DUMP_SAMPLE, seed=0):
+    """A fixed sample of the concatenated, flattened `tensors`: the same flat indices (sorted, drawn from a CPU
+    generator seeded with `seed`) in every run with the same tensor sizes."""
+    flat = torch.cat([t.detach().reshape(-1).float() for t in tensors])
+    if flat.numel() <= n:
+        return flat
+    idx = torch.randint(flat.numel(), (n,), generator=torch.Generator().manual_seed(seed)).sort().values
+    return flat[idx.to(flat.device)]
+
+
+def _timed_outputs(net, result, train):
+    """Device copies of what the last timed step gave its caller.  Inference: the logits.  Train: the loss, and seeded
+    samples of the trained parameters after the optimizer step and of the gradients that step applied (in
+    named_parameters order)."""
+    if not train:
+        return {"logits": result.detach().float().clone()}
+    named = [(n, p) for n, p in net.named_parameters() if not n.startswith("head_dist")]
+    missing = [n for n, p in named if p.grad is None]
+    if missing:
+        raise RuntimeError(f"the timed train step left no gradient for {missing}")
+    params = [p for _, p in named]
+    return {"loss": result.detach().float().clone(),
+            "params_sample": _seeded_sample(params),
+            "grads_sample": _seeded_sample([p.grad for p in params])}
+
+
+def _write_outputs(out_dir, arrays):
+    """DIR/<name>.npy per array, float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 def _other_kernel_rooflines(mel, net, wave, B, ntok, peaks):
@@ -694,7 +733,13 @@ def main():
     ap.add_argument("--graph", type=int, default=1, help="1: replay the step as one CUDA graph (default); 0: eager")
     ap.add_argument("--stock", type=int, default=1,
                     help="1 (default, N=1 only): also time the stock PyTorch-CUDA arms in this run (stock_gpu, vs_stock)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy (float32; "
+                         "train: loss and seeded samples of the updated parameters and their gradients; inference: "
+                         "logits), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

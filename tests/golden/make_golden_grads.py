@@ -6,7 +6,7 @@ Run in the build container only:
 
 Same weights / input / seeds as passt_golden.pt (make_golden.py), so the two fixtures describe one run.  To keep the
 file small, tensors with at most FULL_LIMIT elements are stored whole; larger ones are stored as
-  * 4096 evenly strided samples (`samples`, taken at flat indices `arange(n)[::n // 4096][:4096]`),
+  * 1536 evenly strided samples (`samples`, taken at flat indices `arange(n)[::n // 1536][:1536]`),
   * their double-precision sum, max-abs and L2 norm,
   * 4 random projections <g, r_j> with r_j = randn(generator seeded by crc32(name) + j) -- a whole-tensor check.
 """
@@ -22,8 +22,8 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 from ref_shim import load_reference, quiet  # noqa: E402
 from oracle import passt_oracle as O  # noqa: E402
 
-FULL_LIMIT = 200_000
-N_SAMPLES = 4096
+FULL_LIMIT = 10_000
+N_SAMPLES = 1536
 N_PROJ = 4
 
 

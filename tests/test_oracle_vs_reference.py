@@ -1,35 +1,47 @@
-"""Pin the CPU oracle against the reference implementation itself (imported from /root/reference through the shim).
-Skipped where the reference tree is absent (the GPU box) — there the committed golden fixture takes over."""
+"""Pin the CPU oracle against the reference implementation itself: the reference's outputs on these tests' seeded inputs
+are stored in tests/golden/reference_checks.pt (written by tests/golden/make_reference_checks.py from the unmodified
+reference).  Mel spectrograms are compared bit-exactly through their SHA-256, logits and features bit-exactly;
+gradients element-wise on whole small tensors and strided samples, and on every element through random projections."""
+import hashlib
+import os
+
 import pytest
 import torch
 
-from ref_shim import load_reference, quiet, reference_available
 from oracle import passt_oracle as O
+from util import golden_projections, golden_sample_index
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="reference tree not present")
+PATH = os.path.join(os.path.dirname(__file__), "golden", "reference_checks.pt")
 
 
-def _ref_mel():
-    _, rpre = load_reference()
-    with quiet():
-        return rpre.AugmentMelSTFT(n_mels=128, sr=32000, win_length=800, hopsize=320, n_fft=1024, freqm=48, timem=192,
-                                   htk=False, fmin=0.0, fmax=None, norm=1, fmin_aug_range=10, fmax_aug_range=2000)
+@pytest.fixture(scope="module")
+def G():
+    return torch.load(PATH)
+
+
+@pytest.fixture(scope="module", autouse=True)
+def _reference_thread_count(G):
+    """The reference ran with G["num_threads"] intra-op threads; the CPU matrix products' summation order (the last bits
+    of the logits) depends on that count, so the oracle runs with the same count."""
+    saved = torch.get_num_threads()
+    torch.set_num_threads(G["num_threads"])
+    yield
+    torch.set_num_threads(saved)
 
 
 @pytest.mark.parametrize("training", [False, True])
 @pytest.mark.parametrize("L", [48000, 33001])
-def test_mel_bit_exact(training, L):
-    mel = _ref_mel().train(training)
+def test_mel_bit_exact(G, training, L):
+    ref = G["mel"][f"{'train' if training else 'eval'}_{L}"]
     cfg = O.MelCfg()
     torch.manual_seed(0)
     wave = 0.1 * torch.randn(2, L)
     torch.manual_seed(3)
-    with quiet():
-        ref = mel(wave)
-    torch.manual_seed(3)
     d = O.draw_mel(cfg, training, 2)
     mine = O.mel_frontend(wave, cfg, d, training)
-    assert torch.equal(ref, mine)
+    assert tuple(mine.shape) == ref["shape"] and mine.dtype == torch.float32
+    assert torch.equal(mine.flatten()[golden_sample_index(mine.numel(), G["n_samples"])], ref["samples"])
+    assert hashlib.sha256(mine.contiguous().numpy().tobytes()).hexdigest() == ref["sha256"]
 
 
 def test_mel_banks_match_torchaudio():
@@ -41,16 +53,10 @@ def test_mel_banks_match_torchaudio():
 
 @pytest.mark.parametrize("kw,T", [(dict(s_patchout_t=40, s_patchout_f=4), 1000), (dict(u_patchout=400), 1000),
                                   (dict(s_patchout_t=10, s_patchout_f=3, n_classes=50), 500)])
-def test_net_train_forward_backward_light(kw, T):
+def test_net_train_forward_backward_light(G, kw, T):
     """3-block model (reference lighten_model cut_depth=9): logits, features, draws and gradients."""
-    rp, _ = load_reference()
+    ref = G["net"][",".join(f"{k}={v}" for k, v in sorted(kw.items())) + f",T={T}"]
     cfg12 = O.NetCfg(**kw)
-    with quiet():
-        net = rp.get_model(arch="passt_s_swa_p16_128_ap476", pretrained=False, n_classes=cfg12.n_classes,
-                           u_patchout=cfg12.u_patchout, s_patchout_t=cfg12.s_patchout_t,
-                           s_patchout_f=cfg12.s_patchout_f)
-        net.load_state_dict(O.synth_params(cfg12, 2), strict=True)
-        net = rp.lighten_model(net, cut_depth=9)        # keeps blocks 0, 10, 11
     cfg = O.NetCfg(depth=3, **kw)
     p = {}
     remap = {0: 0, 10: 1, 11: 2}
@@ -64,19 +70,23 @@ def test_net_train_forward_backward_light(kw, T):
     p = {k: v.clone().requires_grad_(True) for k, v in p.items()}
     torch.manual_seed(1)
     x = torch.randn(1, 1, 128, T)
-    net.train()
-    torch.manual_seed(8)
-    with quiet():
-        ref_logits, ref_feat = net(x)
     torch.manual_seed(8)
     d = O.draw_patchout(cfg, 12, (T - 16) // 10 + 1, True)
     lg, ft = O.passt_forward(p, x, cfg, d)
-    assert torch.equal(ref_logits, lg) and torch.equal(ref_feat, ft)
-    ref_logits.sum().backward()
+    assert torch.equal(ref["logits"], lg) and torch.equal(ref["features"], ft)
     lg.sum().backward()
-    ref_grads = dict(net.named_parameters())
-    for k, v in p.items():
-        if k.startswith("head_dist"):
-            assert v.grad is None and ref_grads[k].grad is None
-            continue
-        assert torch.allclose(v.grad, ref_grads[k].grad, rtol=1e-5, atol=1e-7), k
+    assert set(ref["grads"]) == {k for k, v in p.items() if v.grad is not None}
+    for k in ref["no_grad"]:
+        assert p[k].grad is None, k
+    rtol, atol = G["rtol"], G["atol"]
+    for k, rec in ref["grads"].items():
+        g = p[k].grad
+        assert tuple(g.shape) == rec["shape"], k
+        if "full" in rec:
+            assert torch.allclose(g, rec["full"], rtol=rtol, atol=atol), k
+        else:
+            got = g.flatten()[golden_sample_index(g.numel(), G["n_samples"])]
+            assert torch.allclose(got, rec["samples"], rtol=rtol, atol=atol), k
+        # <g - g_ref, r> for unit-variance r is ~ ||g - g_ref||_2, at most the L2 norm of the element-wise envelope
+        pj = golden_projections(k, g, G["n_proj"])
+        assert (pj - rec["proj"]).abs().max().item() <= 5 * rec["env_l2"], k

@@ -3,6 +3,7 @@ tensor-core MMAs (UTCHMMA, .2CTA for cta_group::2), TMEM loads/stores (LDTM / ST
 (UTMALDG / UTMASTG / UTMAREDG) and programmatic dependent launch (ACQBULK / PREEXIT).  Runs `cuobjdump -sass` on the
 in-tree .so; no GPU needed."""
 import collections
+import os
 import re
 import shutil
 import subprocess
@@ -12,13 +13,24 @@ import pytest
 KEYS = ("UTCHMMA", "UTCBAR", "UTMALDG", "UTMASTG", "UTMAREDG", "LDTM", "STTM", "MUFU.EX2", "ACQBULK", "PREEXIT")
 
 
+def _cuobjdump():
+    """cuobjdump from PATH, else from the toolkit of the nvcc the library is built with."""
+    from passt_b200 import build
+    nvcc = shutil.which(build._nvcc())
+    for c in (shutil.which("cuobjdump"), nvcc and os.path.join(os.path.dirname(nvcc), "cuobjdump")):
+        if c and os.path.isfile(c):
+            return c
+    return None
+
+
 @pytest.fixture(scope="module")
 def sass_ops():
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
+    cuobjdump = _cuobjdump()
+    if cuobjdump is None:
+        pytest.skip("cuobjdump not found (neither on PATH nor next to nvcc)")
     from passt_b200 import build
     so = build.build()
-    out = subprocess.run(["cuobjdump", "-sass", str(so)], capture_output=True, text=True, timeout=600).stdout
+    out = subprocess.run([cuobjdump, "-sass", str(so)], capture_output=True, text=True, timeout=600).stdout
     ops = collections.defaultdict(collections.Counter)
     cur = None
     for line in out.splitlines():
